@@ -30,6 +30,9 @@ applications per second (KrylovKit's numops/s, SURVEY §5 "iterations/sec").
   parity   : every arm asserts its Ritz values against the oracle's committed full-size results
              (tests/golden/fullsize.json): <= 1e-10 relative (+ 4 ulp(||A||) floor), numops equal.
   other_configs : BASELINE.json configs 3, 4, 5 measured after the headline, with their own parity evidence.
+  --dump-outputs DIR : what the last timed job returned (Ritz values, ConvergenceInfo, the Ritz and residual vectors
+             at a fixed, seeded sample of rows) as float64 DIR/<name>.npy, about 38 MB in all: the inputs are
+             seeded, so two builds run with the same arguments can be compared output for output.
 
 N > 1: STRONG scaling — the same 1e7-row problem row-sharded over N ranks; halo rows, <v,Av>, the projection
 coefficients and ||w||^2 are exchanged inside the two kernels of a step through the NVLink peer window
@@ -80,7 +83,13 @@ def parse():
                          "GKL mode, run LAST: its kernel had not run on a B200 when the round's GPU budget ended); c5 — the "
                          "configuration BASELINE.json names for 8 GPUs — under torchrun")
     ap.add_argument("--c4-rows", type=int, default=2_000_000, help="rows of config 4's dense matrix (tests use fewer)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed job returned to DIR/<name>.npy (float64, one GPU, --impl ours)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if a.extra is None:
         a.extra = "c2f,c2m,w,c3,c4,c5,c4o" if int(os.environ.get("WORLD_SIZE", "1")) == 1 else "c5"
     return a
@@ -335,6 +344,28 @@ def run_reference(a):
     print(json.dumps(json_safe(line), allow_nan=False, default=str), flush=True)
 
 
+DUMP_ROWS = 1 << 19      # rows of each Ritz / residual vector in a dump: 2 * HOWMANY * 4 MiB + the row list
+
+
+def dump_outputs(out_dir, vals, vecs, info):
+    """Write what an eigsolve call returned to out_dir as float64 .npy files: the Ritz values, the ConvergenceInfo
+    numbers (normres; converged, numiter, numops) and the Ritz and residual vectors at DUMP_ROWS rows drawn with a
+    fixed seed (sample_rows.npy; every row when n is smaller).  Whole vectors at n = 1e7 would be 640 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(vecs[0])
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(SEED).choice(n, DUMP_ROWS, replace=False))
+    arrays = {
+        "ritz_values": np.asarray(vals, dtype=np.float64),
+        "ritz_vectors": np.stack([v.to_host()[rows] for v in vecs]).astype(np.float64),
+        "residuals": np.stack([r.to_host()[rows] for r in info.residual]).astype(np.float64),
+        "normres": np.asarray(info.normres, dtype=np.float64),
+        "counts": np.array([info.converged, info.numiter, info.numops], dtype=np.float64),
+        "sample_rows": rows.astype(np.float64),
+    }
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), arr)
+
+
 def workload_config(a):
     return {"workload": f"eigsolve(Lanczos, :SR, {HOWMANY}) on the {a.nx * a.ny}x{a.nx * a.ny} CSR 5-point "
                         f"Laplacian ({a.nx}x{a.ny} grid, Dirichlet), Float64, krylovdim={a.krylovdim}, "
@@ -353,6 +384,8 @@ def run_ours(a):
     if world != a.gpus:
         if world == 1 and a.gpus > 1:
             raise SystemExit("bench.py --gpus N>1 must be launched with torch.distributed.run (one rank per GPU)")
+    if a.dump_outputs and world > 1:
+        raise SystemExit("bench.py --dump-outputs writes the outputs of a one-GPU run: use it with --gpus 1")
     dist = None
     n = a.nx * a.ny
     orth = {"cgs2": kk.cgs2, "mgs2": kk.mgs2, "cgs": kk.cgs, "mgs": kk.mgs, "mgs2b": kk.mgs2b}[a.orth]
@@ -398,10 +431,11 @@ def run_ours(a):
     lib.b2k_timer_start(ctx.h)
     t0 = time.perf_counter()
     numops = 0
-    for _ in range(a.steps):
+    for i in range(a.steps):
         vals, vecs, info = job()
         numops += info.numops
-        del vecs
+        if i + 1 < a.steps or not a.dump_outputs:
+            del vecs
     ms = C.c_double()
     lib.b2k_timer_stop(ctx.h, C.byref(ms))
     barrier()
@@ -421,6 +455,9 @@ def run_ours(a):
         dist.all_reduce(ll)
         launches = int(ll.item())
     value = numops / t_dev
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, vals, vecs, info)
+        del vecs
     parity = check_parity(a, vals, numops // a.steps, "device-resident path")     # every rank: values are replicated
 
     # roofline of the dominant kernel (fused Gram-Schmidt sweep) + SpMV beside it
@@ -923,6 +960,9 @@ def other_configs(kk, a, rank, world, local_rank, dist):
 
 
 def main():
+    # the tree this runs from may be read-only and stays as the build left it: the modules imported from it below
+    # write no bytecode caches there (nor in the child process of the c4o leg, which runs main() too)
+    sys.dont_write_bytecode = True
     a = parse()
     if os.environ.get("B2K_BENCH_CHILD") == "1":
         # child of other_configs' c4o leg: that one record, as one JSON line, nothing else

@@ -54,6 +54,11 @@ def test_failing_extra_config_becomes_a_record(monkeypatch, capsys):
         B200Context=FakeCtx,
         B200CSR=types.SimpleNamespace(stencil_free=fail, stencil=fail),
         cgs2=None, mgs2=None, cgs=None, mgs=None, mgs2b=None)
+    # the legs that use the real package fail too, also where a GPU is present: tools/run_configs.py (in this
+    # process) cannot create a context, and the c4o child process sees no CUDA device
+    import krylovkit_jl_b200 as kk
+    monkeypatch.setattr(kk, "B200Context", fail)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     out = bench.other_configs(fake, a, 0, 1, 0, None)
     assert set(out) == {"c2_matrix_free", "c2_reference_default_orth", "widened_solvers", "c3", "c4", "c5", "c4_onepass"}
     for name, rec in out.items():
@@ -136,30 +141,36 @@ def test_onepass_extra_runs_on_the_simulator(monkeypatch):
 
 def test_onepass_extra_is_isolated_in_a_child_process(monkeypatch):
     """bench.other_configs 'c4o' without B2K_BENCH_CHILD spawns `bench.py --extra c4o` as a child and turns whatever
-    happens there into a record: here (no CUDA device) the child's context creation fails, the child still prints its
-    record, and the parent carries it — the parent itself never touches the one-pass kernel."""
+    happens there into a record: here (the child sees no CUDA device) the child's context creation fails, the child
+    still prints its record, and the parent carries it — the parent itself never touches the one-pass kernel."""
     bench = _load_bench()
     monkeypatch.setattr(sys, "argv", ["bench.py", "--extra", "c4o", "--c4-rows", "4000"])
     monkeypatch.delenv("B2K_BENCH_CHILD", raising=False)
     monkeypatch.delenv("WORLD_SIZE", raising=False)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     a = bench.parse()
     out = bench.other_configs(types.SimpleNamespace(_lib=types.SimpleNamespace(load=lambda: None)), a, 0, 1, 0, None)
     rec = out["c4_onepass"]
     assert rec["ok"] is False and "error" in rec and ("B200Error" in rec["error"] or "CUDA" in rec["error"] or "cuda" in rec["error"])
 
 
-def test_headline_path_runs_on_the_simulator_and_prints_the_contract(monkeypatch, capsys):
+def test_headline_path_runs_on_the_simulator_and_prints_the_contract(monkeypatch, capsys, tmp_path):
     """bench.run_ours end to end on tests/hostsim.py at a small size — the resident job, the host-buffer (e2e) leg with
     its pinned buffers, the per-kernel profile and the assembly of the one JSON line — so that the host code of the
     headline is exercised on a box without a GPU.  The line must parse STRICTLY (no NaN / Infinity tokens) and carry
-    the keys of the bench contract; the Ritz values of both legs must agree with the oracle on the same (A, x0)."""
+    the keys of the bench contract; the Ritz values of both legs must agree with the oracle on the same (A, x0).
+    --dump-outputs (with fewer sampled rows than n) writes what the last timed job returned: float64 arrays that agree
+    with the oracle's values, vectors and residuals at the sampled rows."""
     import json
+    import numpy as np
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import hostsim
     from oracle import krylov_oracle as ko
     bench = _load_bench()
+    dump = tmp_path / "outputs"
+    monkeypatch.setattr(bench, "DUMP_ROWS", 500)
     monkeypatch.setattr(sys, "argv", ["bench.py", "--nx", "40", "--ny", "30", "--krylovdim", "12", "--cycles", "3", "--steps", "2",
-                                      "--warmup", "1", "--no-cpu-baseline", "--extra", ""])
+                                      "--warmup", "1", "--no-cpu-baseline", "--extra", "", "--dump-outputs", str(dump)])
     monkeypatch.delenv("WORLD_SIZE", raising=False)
     monkeypatch.delenv("B2K_BENCH_CHILD", raising=False)
     a = bench.parse()
@@ -177,10 +188,20 @@ def test_headline_path_runs_on_the_simulator_and_prints_the_contract(monkeypatch
     assert line["n_gpus"] == 1 and line["steps"] == 2 and line["dtype"] == "f64" and line["gpu_launches"] > 0
     assert line["numops_per_step"] == 12 + 2 * (12 - (3 * 12) // 5) and line["value"] > 0
     assert line["e2e"]["h2d_bytes_per_step"] > 0 and line["e2e"]["d2h_bytes_per_step"] > 0 and line["e2e"]["value"] > 0
-    ov, _, oi = ko.eigsolve_lanczos(ko.stencil_matrix(40, 30), ko.splitmix_vector(bench.SEED, 1200), 4, "SR", krylovdim=12,
-                                    maxiter=3, tol=0.0, orth=ko.Orth(ko.CGS2))
+    ov, ovecs, oi = ko.eigsolve_lanczos(ko.stencil_matrix(40, 30), ko.splitmix_vector(bench.SEED, 1200), 4, "SR", krylovdim=12,
+                                        maxiter=3, tol=0.0, orth=ko.Orth(ko.CGS2))
     assert oi["numops"] == line["numops_per_step"]
     assert max(abs(x - y) for x, y in zip(line["ritz_values"], ov[:4])) < 1e-10
+    got = {p.stem: np.load(p) for p in dump.iterdir()}
+    assert set(got) == {"ritz_values", "ritz_vectors", "residuals", "normres", "counts", "sample_rows"}
+    assert all(x.dtype == np.float64 for x in got.values())
+    rows = got["sample_rows"].astype(np.int64)
+    assert len(rows) == 500 and np.all(np.diff(rows) > 0) and rows[-1] < 1200
+    assert got["ritz_values"].tolist() == line["ritz_values"]
+    assert got["counts"].tolist() == [oi["converged"], oi["numiter"], oi["numops"]]
+    np.testing.assert_allclose(got["normres"], oi["normres"][:4], rtol=1e-8, atol=1e-14)
+    np.testing.assert_allclose(got["ritz_vectors"], np.stack([v[rows] for v in ovecs[:4]]), atol=1e-10)
+    np.testing.assert_allclose(got["residuals"], np.stack([r[rows] for r in oi["residual"][:4]]), atol=1e-10)
 
 
 def test_json_safe_makes_any_record_strictly_parseable():

@@ -4,11 +4,10 @@ product path fails loudly (no CPU fallback) when no device is present."""
 import os
 import re
 import subprocess
+import sys
 
 import numpy as np
-import pytest
 
-import krylovkit_jl_b200 as kk
 from krylovkit_jl_b200 import _lib as L
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -47,16 +46,27 @@ def test_abi_version_and_status_codes():
         assert m and int(m.group(1)) == val
 
 
+NO_DEVICE_CHILD = """
+import numpy as np
+import pytest
+import scipy.sparse as sp
+import krylovkit_jl_b200 as kk
+with pytest.raises(kk.B200Error, match="no CPU fallback"):
+    kk.B200Context(100, 8)
+with pytest.raises(kk.B200Error):
+    kk.eigsolve(sp.identity(10, format="csr"), np.ones(10), 1, "SR", kk.Lanczos(krylovdim=5))
+print("no fallback: ok")
+"""
+
+
 def test_no_cpu_fallback_without_device():
-    from conftest import HAVE_GPU
-    if HAVE_GPU:
-        pytest.skip("a GPU is present")
-    with pytest.raises(kk.B200Error, match="no CPU fallback"):
-        kk.B200Context(100, 8)
-    import numpy as np
-    import scipy.sparse as sp
-    with pytest.raises(kk.B200Error):
-        kk.eigsolve(sp.identity(10, format="csr"), np.ones(10), 1, "SR", kk.Lanczos(krylovdim=5))
+    """In a process that sees no CUDA device, context creation and the host-buffer eigsolve raise B200Error instead
+    of computing on the CPU.  The child process hides the devices, so a machine with a GPU checks this too."""
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    flags = ["-s"] if sys.flags.no_user_site else []
+    r = subprocess.run([sys.executable, *flags, "-c", NO_DEVICE_CHILD], cwd=ROOT, env=env, capture_output=True,
+                       text=True, timeout=300)
+    assert r.returncode == 0 and "no fallback: ok" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
 
 
 def test_product_never_imports_oracle():
